@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the SVSDF cost+gradient hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic input: one evaluation of
 TrajOptimizer::addSaftyPenaOnSweptVolumeParallelTrueSDF (reference: back_end_optimizer.hpp:774-869) over the
@@ -231,6 +231,16 @@ def cpu_baseline(sc, reps: int = 3):
             "builds": tried, "seconds_per_eval": sec}
 
 
+def dump_outputs(outdir: str, cost, grad_T, grad_coeffs, n_inside=None):
+    """The arrays a caller of the timed path receives, one float64 .npy each (a few hundred bytes for config 2)."""
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {"cost": np.atleast_1d(cost), "grad_T": grad_T, "grad_coeffs": grad_coeffs}
+    if n_inside is not None:
+        arrays["n_inside"] = np.atleast_1d(n_inside)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64).reshape(-1))
+
+
 def run_reference(args):
     rank, world, _ = dist_env()
     if rank != 0:
@@ -241,8 +251,10 @@ def run_reference(args):
         cp.eval_once()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cp.eval_once()
+        res = cp.eval_once()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res[0], res[1], res[2])
     value = sc.P * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -271,7 +283,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-lbfgs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (cost, gradients, inside count) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -328,7 +344,9 @@ def main():
         pr, c, cc = problem_of(s_)
         flush.zero_()  # flush L2 between timed iterations (untimed)
         torch.cuda.synchronize()
-        ms, _ = c.cost_grad_device(pr.T, cc, repeats=1, fetch=False)  # CUDA events on the launching stream
+        # every step copies its result to the host after the stop event; fetch only hands the last one to Python
+        fetch = bool(args.dump_outputs) and s_ == args.steps - 1
+        ms, out = c.cost_grad_device(pr.T, cc, repeats=1, fetch=fetch)  # CUDA events on the launching stream
         ms_steps.append(ms)
         if c is ctx:
             outer_ms.append(c.last_kernel_ms()[1])
@@ -372,6 +390,8 @@ def main():
     d2h = 8 * (1 + 19 * N_PIECES + 1)
 
     extra = {}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out[0], out[1 + 18 * N_PIECES:1 + 19 * N_PIECES], out[1:1 + 18 * N_PIECES], out[1 + 19 * N_PIECES])
     if rank == 0:
         # ---- roofline of the dominant kernel (k_outer), FP64 non-tensor pipe ----
         ctx.executed_evals(True)

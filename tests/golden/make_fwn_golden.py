@@ -67,6 +67,50 @@ def ref_fwn_tree(V, F, order=2):
     return ch, data
 
 
+BRANCH_MESHES = ["synthetic_star", "two_faces", "seven_faces", "grid_900", "degenerate_duplicates"]
+
+
+def branch_case(mesh):
+    """(V, F, Q) of a mesh that exercises one branch of the hierarchy builder: 2 items, the exhaustive <= 6 split, the sorted
+    <= 32 split, the 16-span binning, coincident centres (nthElement fallback)."""
+    rng = np.random.default_rng(9)
+    if mesh == "synthetic_star":
+        V, F = scenes.extrude_outline(scenes.star_outline(n_per_edge=4))
+    elif mesh in ("two_faces", "seven_faces"):
+        nf = 2 if mesh == "two_faces" else 7
+        V = rng.uniform(-2, 2, size=(3 * nf, 3))
+        F = np.arange(3 * nf, dtype=np.int32).reshape(nf, 3)
+    elif mesh == "grid_900":
+        n = 16
+        xs, ys = np.meshgrid(np.linspace(-3, 3, n), np.linspace(-2, 2, n))
+        V = np.c_[xs.ravel(), ys.ravel(), 0.3 * np.sin(xs.ravel() * 2.0) * np.cos(ys.ravel())]
+        F = []
+        for i in range(n - 1):
+            for j in range(n - 1):
+                a = i * n + j
+                F += [[a, a + 1, a + n + 1], [a, a + n + 1, a + n]]
+        F = np.asarray(F, dtype=np.int32)
+    else:  # many faces sharing one centre: the span partition cannot split them
+        base = rng.uniform(-1, 1, size=(3, 3))
+        V = np.concatenate([base * (1.0 + 0.0 * k) for k in range(40)] + [rng.uniform(-2, 2, size=(30, 3))])
+        F = np.arange(len(V), dtype=np.int32).reshape(-1, 3)
+    lo, hi = V.min(axis=0) - 1.5, V.max(axis=0) + 1.5
+    Q = np.zeros((3000, 3))
+    Q[:, :2] = rng.uniform(lo[:2], hi[:2], size=(3000, 2))
+    Q[1500:] = rng.uniform(lo, hi, size=(1500, 3))
+    return V, F, Q
+
+
+def branch_fixture():
+    """fwn_ref_branches.npz: the reference's winding numbers and hierarchy for the meshes of branch_case."""
+    out = {}
+    for mesh in BRANCH_MESHES:
+        V, F, Q = branch_case(mesh)
+        out[mesh + "_w_ref"] = ref_fwn(V, F, Q)
+        out[mesh + "_tree_children"], out[mesh + "_tree_data"] = ref_fwn_tree(V, F)
+    np.savez_compressed(os.path.join(HERE, "fwn_ref_branches.npz"), **out)
+
+
 def main():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"])
     rng = np.random.Generator(np.random.MT19937(20240511))
@@ -90,6 +134,7 @@ def main():
     Q[2000:] = rng2.uniform(lo, hi, size=(1000, 3))
     np.savez_compressed(os.path.join(HERE, "fwn_ref_sdarc.npz"), sdArc_V=V, sdArc_F=F, sdArc_Q=Q, sdArc_w_ref=ref_fwn(V, F, Q),
                         sdArc_tree_children=ref_fwn_tree(V, F)[0])
+    branch_fixture()
     for k, v in out.items():
         print(k, v.shape, v.dtype)
 

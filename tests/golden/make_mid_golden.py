@@ -39,8 +39,29 @@ def problem(N, seed):
     return init_s, final_s, Q, rots, x
 
 
+def perturbed_cases():
+    """(key, N, cfg, init_s, final_s, Q, rots, x) at seeded perturbations of two problems, both parameter sets."""
+    rng = np.random.default_rng(3)
+    for N in (4, 9):
+        init_s, final_s, Q, rots, x = problem(N, 500 + N)
+        for cname, over in CONFIGS.items():
+            cfg = api.mid_default_config(**over)
+            for j in range(3):
+                yield f"{cname}_N{N}_{j}_", N, cfg, init_s, final_s, Q, rots, x + rng.normal(0, 0.2, x.shape)
+
+
+def perturbed_fixture():
+    """ref_mid_perturbed.npz: cost and gradient of the reference's OriTraj::costFunction at perturbed_cases."""
+    out = {}
+    for k, N, cfg, init_s, final_s, Q, rots, x in perturbed_cases():
+        i_s, f_s, q, r, _ = api._mid_args(init_s, final_s, Q, rots)
+        out[k + "cost"], out[k + "grad"] = R.mid_cost(cfg, N, i_s, f_s, q, r, x)
+    np.savez_compressed(os.path.join(HERE, "ref_mid_perturbed.npz"), **out)
+
+
 def main():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref_path"], stdout=subprocess.DEVNULL)
+    perturbed_fixture()
     out = {}
     for cname, over in CONFIGS.items():
         cfg = api.mid_default_config(**over)

@@ -11,6 +11,7 @@ algorithm that the CUDA kernels implement — so the CUDA path can be compared w
 Fixtures (inputs + reference outputs; the reference tree cannot travel to the GPU box, these can):
   ref_pin_shapes.npz  16 registry shapes + Circle + Polygon fallback x 2 body-frame pre-transforms: getonlySDF on 2 000
                       points, getonlyGrad1 on 400, BasicShape::initShape byte kernels (17 x 17 x 18 yaws)
+  ref_pin_sample.npz  seeded samples of larger inputs (sample_fixture)
   ref_pin_path.npz    three scenes (config 1: star / N = 8 / 2 000 points; a 400-point scene with ~6 % interior points;
                       sdHorseshoe / N = 16 / 1 500 points): Trajectory<5>::getPos/getVel samples, per point
                       getTrueSDFofSweptVolume<true> (sdf, t*, gradient), the accumulating penalty loop (cost, gradT,
@@ -56,8 +57,58 @@ def shapes_fixture():
             yaw, cells, byt = R.shape_kernels(s, 17, 18, 1.0, 0.0, variant=v)
             out[f"kyaw_{v}_{s}"] = yaw
             out[f"kbytes_{v}_{s}"] = byt
-    np.savez_compressed(os.path.join(HERE, "ref_pin_shapes.npz"), **out)
+    save_fixture("ref_pin_shapes.npz", out)
     print("ref_pin_shapes.npz", len(out), "arrays")
+
+
+def save_fixture(name, out):
+    """Most shapes call no libm function, so both builds agree bit for bit: such a "portable" array is stored once, as "glibc"."""
+    for k in [k for k in out if "_portable_" in k]:
+        a, b = out[k], out[k.replace("_portable_", "_glibc_")]
+        if a.dtype == b.dtype and a.shape == b.shape and a.tobytes() == b.tobytes():
+            del out[k]
+    np.savez_compressed(os.path.join(HERE, name), **out)
+
+
+def load_fixture(name):
+    """A fixture written by save_fixture, with every "portable" array present again."""
+    g = dict(np.load(os.path.join(HERE, name)))
+    for k in [k for k in g if "_glibc_" in k]:
+        g.setdefault(k.replace("_glibc_", "_portable_"), g[k])
+    return g
+
+
+def shapes_1e5_points():
+    """The 1e5 body-frame points of the sampled shape test, two pre-transforms, and the seeded sample stored of them."""
+    rng = np.random.default_rng(77)
+    n = 100_000
+    rel = np.c_[rng.uniform(-9.0, 9.0, (n, 2)), rng.uniform(-1.0, 1.0, n)]
+    pick = np.random.default_rng(78)
+    return rel, [(0.0, 0.0, 0.0), (-0.4, 0.15, -70.0)], np.sort(pick.choice(n, 512, replace=False)), np.sort(pick.choice(5000, 128, replace=False))
+
+
+def scene_20k():
+    return scenes.make_scene("star", 8, 20_000, seed_map=991)
+
+
+def sample_fixture():
+    """ref_pin_sample.npz: the reference's outputs at a seeded sample of larger inputs (shapes_1e5_points: getonlySDF on 512 of 1e5
+    points, getonlyGrad1 on 128 of 5 000; scene_20k: getTrueSDFofSweptVolume<true> of the portable build on 2 000 of 20 000 points)."""
+    rel, pres, si, gi = shapes_1e5_points()
+    out = {}
+    for v in VARIANTS:
+        for ip, pp in enumerate(pres):
+            for s in SHAPES:
+                out[f"sdf_{v}_{ip}_{s}"] = R.shape_sdf(s, rel[si], pp, variant=v)
+        for s in SHAPES:
+            out[f"grad1_{v}_{s}"] = R.shape_grad1(s, rel[:5000][gi], variant=v)
+    sc = scene_20k()
+    idx = np.sort(np.random.default_rng(992).choice(sc.P, 2000, replace=False))
+    ref = R.RefPath("star", weight_p=sc.weight_p, safety_hor=sc.safety_hor, rho=sc.rho, threads=8, variant="portable")
+    ref.set_traj(sc.T, sc.coeffs_colmajor())
+    out["scene20k_idx"] = idx
+    out["scene20k_sdf"], out["scene20k_tstar"], out["scene20k_grad"] = ref.query(np.c_[sc.points[idx, :2], np.zeros(len(idx))])
+    save_fixture("ref_pin_sample.npz", out)
 
 
 def path_fixture():
@@ -112,3 +163,4 @@ if __name__ == "__main__":
         R.build()
     shapes_fixture()
     path_fixture()
+    sample_fixture()

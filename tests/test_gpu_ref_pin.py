@@ -8,6 +8,7 @@ path (strict build, through the C ABI) must reproduce every per-point output of 
 Against the "glibc" variant (the reference as it runs) the known libm noise floor applies (see test_gpu_parity.py).
 """
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -17,6 +18,8 @@ from implicit_svsdf_planner_b200 import api
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
+sys.path.insert(0, GOLD)
+import make_ref_pin_golden as mk  # noqa: E402  (fixture loader; its reference calls are not used here)
 
 
 def bits_differ(a, b):
@@ -31,7 +34,7 @@ def bits_differ(a, b):
 
 @pytest.fixture(scope="module")
 def gshapes():
-    return np.load(os.path.join(GOLD, "ref_pin_shapes.npz"))
+    return mk.load_fixture("ref_pin_shapes.npz")
 
 
 @pytest.fixture(scope="module")
@@ -105,22 +108,13 @@ def test_path_is_bitwise_the_reference_code(gpath, key):
     ctx.close()
 
 
-def test_live_reference_library_on_this_box_agrees_at_20k_points(gpath):
-    """When the compiled reference travels with the snapshot (oracle/_ref/*.so), run it HERE on fresh seeded points, not
-    only on the committed fixture."""
-    from oracle import ref_py
-
-    if not ref_py.available("portable"):
-        pytest.skip("oracle/_ref/libref_path_portable.so not present")
-    from implicit_svsdf_planner_b200 import scenes
-
-    sc = scenes.make_scene("star", 8, 20_000, seed_map=991)
-    co = sc.coeffs_colmajor()
-    p0 = np.c_[sc.points[:, :2], np.zeros(sc.P)]
-    ref = ref_py.RefPath("star", weight_p=sc.weight_p, safety_hor=sc.safety_hor, rho=sc.rho, threads=os.cpu_count() or 8, variant="portable")
-    ref.set_traj(sc.T, co)
-    rs, rt, rg = ref.query(p0)
+def test_live_reference_library_on_this_box_agrees_at_20k_points():
+    """A scene of 20 000 fresh seeded points, not only the committed path fixture: every point is queried, a seeded sample of
+    2 000 is compared with what the reference's portable build computes there (ref_pin_sample.npz)."""
+    g = mk.load_fixture("ref_pin_sample.npz")
+    sc = mk.scene_20k()
+    idx = g["scene20k_idx"]
     ctx = api.Context("star", weight_p=sc.weight_p, safety_hor=sc.safety_hor, rho=sc.rho, strict_fp=True)
-    s, t, g, _ = ctx.query(sc.T, co, p0)
-    assert bits_differ(s, rs) + bits_differ(t, rt) + bits_differ(g, rg) == 0
+    s, t, gr, _ = ctx.query(sc.T, sc.coeffs_colmajor(), np.c_[sc.points[:, :2], np.zeros(sc.P)])
+    assert bits_differ(s[idx], g["scene20k_sdf"]) + bits_differ(t[idx], g["scene20k_tstar"]) + bits_differ(gr[idx], g["scene20k_grad"]) == 0
     ctx.close()

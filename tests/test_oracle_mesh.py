@@ -11,7 +11,6 @@ import pytest
 from implicit_svsdf_planner_b200 import api, scenes
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_FWN = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "libref_fwn.so")
 
 
 def cube(h=1.0):
@@ -147,43 +146,19 @@ def test_winding_number_is_bitwise_the_reference_fwn_golden(oracle_mod, name):
     assert np.abs(sdf - oracle_mod.mesh_eval(m, Q, "sdf_exact"))[far].max() <= 1.0e-2 * np.abs(sdf[far]).max()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_FWN), reason="oracle/_ref/libref_fwn.so not built (needs /root/reference)")
 @pytest.mark.parametrize("mesh", ["synthetic_star", "two_faces", "seven_faces", "grid_900", "degenerate_duplicates"])
 def test_reference_fwn_live_tree_coefficients_and_values(oracle_mod, mesh):
-    """Against the reference's compiled code on this machine, on meshes that exercise every branch of the builder: 2 items,
-    the exhaustive <= 6 split, the sorted <= 32 split, the 16-span binning, coincident centres (nthElement fallback)."""
+    """Against what the reference's compiled code computes (tests/golden/fwn_ref_branches.npz, make_fwn_golden.branch_fixture)
+    on meshes that exercise every branch of the builder: 2 items, the exhaustive <= 6 split, the sorted <= 32 split, the
+    16-span binning, coincident centres (nthElement fallback)."""
     import sys
 
     sys.path.insert(0, os.path.join(HERE, "golden"))
     import make_fwn_golden as mk
 
-    rng = np.random.default_rng(9)
-    if mesh == "synthetic_star":
-        V, F = scenes.extrude_outline(scenes.star_outline(n_per_edge=4))
-    elif mesh in ("two_faces", "seven_faces"):
-        nf = 2 if mesh == "two_faces" else 7
-        V = rng.uniform(-2, 2, size=(3 * nf, 3))
-        F = np.arange(3 * nf, dtype=np.int32).reshape(nf, 3)
-    elif mesh == "grid_900":
-        n = 16
-        xs, ys = np.meshgrid(np.linspace(-3, 3, n), np.linspace(-2, 2, n))
-        V = np.c_[xs.ravel(), ys.ravel(), 0.3 * np.sin(xs.ravel() * 2.0) * np.cos(ys.ravel())]
-        F = []
-        for i in range(n - 1):
-            for j in range(n - 1):
-                a = i * n + j
-                F += [[a, a + 1, a + n + 1], [a, a + n + 1, a + n]]
-        F = np.asarray(F, dtype=np.int32)
-    else:  # many faces sharing one centre: the span partition cannot split them
-        base = rng.uniform(-1, 1, size=(3, 3))
-        V = np.concatenate([base * (1.0 + 0.0 * k) for k in range(40)] + [rng.uniform(-2, 2, size=(30, 3))])
-        F = np.arange(len(V), dtype=np.int32).reshape(-1, 3)
-    lo, hi = V.min(axis=0) - 1.5, V.max(axis=0) + 1.5
-    Q = np.zeros((3000, 3))
-    Q[:, :2] = rng.uniform(lo[:2], hi[:2], size=(3000, 2))
-    Q[1500:] = rng.uniform(lo, hi, size=(1500, 3))
-    w_ref = mk.ref_fwn(V, F, Q)
-    rc, rd = mk.ref_fwn_tree(V, F)
+    V, F, Q = mk.branch_case(mesh)
+    g = np.load(os.path.join(HERE, "golden", "fwn_ref_branches.npz"))
+    w_ref, rc, rd = g[mesh + "_w_ref"], g[mesh + "_tree_children"], g[mesh + "_tree_data"]
     ch, data, w_host = api.mesh_fwn_host(V, F, Q)
     assert np.array_equal(ch, rc)
     assert np.array_equal(data.view(np.uint32), rd.view(np.uint32))

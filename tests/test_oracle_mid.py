@@ -92,21 +92,13 @@ def test_own_solver_reaches_at_least_what_the_reference_reaches(gold, cname, N):
 
 
 def test_live_reference_library_when_present(gold):
-    from oracle import ref_py as R
-
-    if not R.mid_available():
-        pytest.skip("oracle/_ref/libref_mid.so not present")
-    rng = np.random.default_rng(3)
-    for N in (4, 9):
-        init_s, final_s, Q, rots, x = mk.problem(N, 500 + N)
-        for over in mk.CONFIGS.values():
-            cfg = api.mid_default_config(**over)
-            i_s, f_s, q, r, _ = api._mid_args(init_s, final_s, Q, rots)
-            for _ in range(3):
-                xx = x + rng.normal(0, 0.2, x.shape)
-                c, g = api.mid_cost(init_s, final_s, Q, rots, xx, cfg)
-                cr, gr = R.mid_cost(cfg, N, i_s, f_s, q, r, xx)
-                assert abs(c - cr) <= 1e-13 * abs(cr) and np.linalg.norm(g - gr) <= 1e-11 * np.linalg.norm(gr)
+    """Cost and gradient away from the golden x: the reference's values at seeded perturbations of two further problems
+    (tests/golden/ref_mid_perturbed.npz, make_mid_golden.perturbed_fixture)."""
+    ref = np.load(os.path.join(HERE, "golden", "ref_mid_perturbed.npz"))
+    for k, N, cfg, init_s, final_s, Q, rots, xx in mk.perturbed_cases():
+        c, g = api.mid_cost(init_s, final_s, Q, rots, xx, cfg)
+        cr, gr = float(ref[k + "cost"]), ref[k + "grad"]
+        assert abs(c - cr) <= 1e-13 * abs(cr) and np.linalg.norm(g - gr) <= 1e-11 * np.linalg.norm(gr), k
 
 
 def test_mid_end_argument_checks():

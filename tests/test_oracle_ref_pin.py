@@ -7,19 +7,23 @@ Two layers:
     BIT — shape values and FD gradients for all 18 functors, initShape byte kernels, Piece<5>/Trajectory<5> samples,
     getTrueSDFofSweptVolume (sdf, t*, gradient; outside and GSIP points), smoothedL1, tau<->T — and every summed quantity
     (cost, gradC, gradT, f, g, MINCO) to summation-order rounding;
-  * live tests (when the .so files are present: this container and the GPU box): 1e5 random points per shape, and the
-    proof that the one arithmetic freedom of the Eigen stand-in (association order of reductions) cannot move any pinned
+  * 1e5 random points per shape against a seeded sample of the reference's values (ref_pin_sample.npz);
+  * live tests (when the .so files are present, i.e. where the reference was compiled): the fixtures are what the reference
+    produces, and the proof that the one arithmetic freedom of the Eigen stand-in (association order of reductions) cannot move any pinned
     per-point output: three builds with three orders agree bit for bit.
 Variant mapping: reference "glibc" <-> oracle "glibc"; reference "portable" (its libm calls redirected to the pinned
 fdlibm sin/cos/atan2) <-> oracle "default" (the variant the CUDA kernels are bit-identical to).
 """
 import os
+import sys
 
 import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
+sys.path.insert(0, GOLD)
+import make_ref_pin_golden as mk  # noqa: E402  (fixture loader; its reference calls are not used here)
 PAIRS = [("glibc", "glibc"), ("portable", "default")]  # (reference variant, oracle variant)
 
 
@@ -32,7 +36,7 @@ def bits_differ(a, b):
 
 @pytest.fixture(scope="module")
 def gshapes():
-    return np.load(os.path.join(GOLD, "ref_pin_shapes.npz"))
+    return mk.load_fixture("ref_pin_shapes.npz")
 
 
 @pytest.fixture(scope="module")
@@ -177,17 +181,17 @@ def _ref():
 
 @pytest.mark.parametrize("rv,ov", PAIRS)
 def test_live_shapes_1e5_points_bitwise(oracle_mod, gshapes, rv, ov):
-    R = _ref()
-    rng = np.random.default_rng(77)
-    n = 100_000
-    rel = np.c_[rng.uniform(-9.0, 9.0, (n, 2)), rng.uniform(-1.0, 1.0, n)]
-    for pp in [(0.0, 0.0, 0.0), (-0.4, 0.15, -70.0)]:
+    """1e5 fresh random points per shape; a seeded sample of them is compared with the reference's values there
+    (ref_pin_sample.npz)."""
+    g = mk.load_fixture("ref_pin_sample.npz")
+    rel, pres, si, gi = mk.shapes_1e5_points()
+    for ip, pp in enumerate(pres):
         for s in gshapes["shapes"]:
             s = str(s)
-            assert bits_differ(_orc_shape(oracle_mod, ov, s, rel, pp, "sdf"), R.shape_sdf(s, rel, pp, variant=rv)) == 0, (s, pp)
+            assert bits_differ(_orc_shape(oracle_mod, ov, s, rel, pp, "sdf")[si], g[f"sdf_{rv}_{ip}_{s}"]) == 0, (s, pp)
     for s in gshapes["shapes"]:
         s = str(s)
-        assert bits_differ(_orc_shape(oracle_mod, ov, s, rel[:5000], (0.0, 0.0, 0.0), "grad"), R.shape_grad1(s, rel[:5000], variant=rv)) == 0, s
+        assert bits_differ(_orc_shape(oracle_mod, ov, s, rel[:5000], (0.0, 0.0, 0.0), "grad")[gi], g[f"grad1_{rv}_{s}"]) == 0, s
 
 
 def test_live_fixture_is_what_the_reference_code_produces(gpath, gshapes):
