@@ -84,6 +84,37 @@ class LbfgsParams(C.Structure):
     ]
 
 
+class ScaleSpec(C.Structure):
+    """svsdf_scale: body scale S(t) = diag(s_x(t), s_y(t), 1), per axis s = c, then s = s + sin(w_k t + phi_k) a_k."""
+    _fields_ = [
+        ("n_terms", C.c_int * 2),
+        ("c", C.c_double * 2),
+        ("a", (C.c_double * 4) * 2),
+        ("w", (C.c_double * 4) * 2),
+        ("phi", (C.c_double * 4) * 2),
+        ("exact_yaw_grad", C.c_int),
+    ]
+
+
+# the reference's commented getScale example (sw_manager.hpp:499-502): diag(0.8 + sin(1.5 t - 1.0) 0.6, sin(1.8 t) 0.4 + 0.8, 1)
+REFERENCE_SCALE_EXAMPLE = dict(x=(0.8, [(0.6, 1.5, -1.0)]), y=(0.8, [(0.4, 1.8, 0.0)]))
+
+
+def scale_spec(x=None, y=None, exact_yaw_grad=False) -> ScaleSpec:
+    """ScaleSpec from per-axis (c, [(a, w, phi), ...]) tuples (up to 4 terms; None: the constant 1)."""
+    s = ScaleSpec()
+    for ax, spec in enumerate((x, y)):
+        c, terms = (1.0, []) if spec is None else (spec[0], list(spec[1]))
+        if len(terms) > 4:
+            raise ValueError("at most 4 sine terms per axis")
+        s.n_terms[ax] = len(terms)
+        s.c[ax] = float(c)
+        for k, (a, w, phi) in enumerate(terms):
+            s.a[ax][k], s.w[ax][k], s.phi[ax][k] = float(a), float(w), float(phi)
+    s.exact_yaw_grad = 1 if exact_yaw_grad else 0
+    return s
+
+
 class OptStats(C.Structure):
     _fields_ = [
         ("final_cost", C.c_double),
@@ -101,7 +132,7 @@ EVAL_T = C.CFUNCTYPE(C.c_double, C.c_void_p, dp, dp, C.c_int)
 # every symbol include/svsdf.h declares (tests check the library exports all of them)
 EXPORTED_SYMBOLS = [
     "svsdf_default_config", "svsdf_create", "svsdf_destroy", "svsdf_last_error", "svsdf_shape_id", "svsdf_shape_bound_radius",
-    "svsdf_set_points", "svsdf_set_points_device", "svsdf_set_traj", "svsdf_query", "svsdf_cost_grad",
+    "svsdf_set_points", "svsdf_set_points_device", "svsdf_set_traj", "svsdf_set_scale", "svsdf_query", "svsdf_cost_grad",
     "svsdf_set_boundary", "svsdf_evaluate", "svsdf_last_costs", "svsdf_get_traj", "svsdf_default_lbfgs_params",
     "svsdf_optimize", "svsdf_optimize_batch", "svsdf_cost_grad_batch", "svsdf_minco_forward", "svsdf_minco_propagate", "svsdf_forward_T", "svsdf_backward_T",
     "svsdf_shape_sdf", "svsdf_shape_grad1", "svsdf_cost_grad_device", "svsdf_kernel_launches",
@@ -142,6 +173,7 @@ def lib():
     L.svsdf_set_points.argtypes = [vp, dp, C.c_int64, C.c_int]
     L.svsdf_set_points_device.argtypes = [vp, vp, C.c_int64]
     L.svsdf_set_traj.argtypes = [vp, C.c_int, dp, dp]
+    L.svsdf_set_scale.argtypes = [vp, C.POINTER(ScaleSpec)]
     L.svsdf_query.argtypes = [vp, C.c_int, dp, dp, C.c_int64, dp, dp, dp, dp, C.POINTER(C.c_int), C.c_int]
     L.svsdf_cost_grad.argtypes = [vp, C.c_int, dp, dp, dp, dp, dp]
     L.svsdf_set_boundary.argtypes = [vp, dp, dp, C.c_int]
@@ -465,6 +497,14 @@ class Context:
         T = _f64(T)
         c = _f64(coeffs_colmajor).reshape(-1)
         self._ck(lib().svsdf_set_traj(self.h, T.shape[0], _p(T), _p(c)), "svsdf_set_traj")
+
+    def set_scale(self, x=None, y=None, exact_yaw_grad=False, spec: "ScaleSpec | None" = None):
+        """Deformable robot: body scale S(t) = diag(s_x(t), s_y(t), 1) on this context's cost path (svsdf_set_scale).
+        x, y = (c, [(a, w, phi), ...]) per axis, or a ready ScaleSpec; no arguments return to the rigid body.
+        e.g. ctx.set_scale(**REFERENCE_SCALE_EXAMPLE)."""
+        if spec is None and (x is not None or y is not None):
+            spec = scale_spec(x, y, exact_yaw_grad)
+        self._ck(lib().svsdf_set_scale(self.h, C.byref(spec) if spec is not None else None), "svsdf_set_scale")
 
     def query(self, T, coeffs_colmajor, pts, outer_only=False):
         T = _f64(T)

@@ -211,6 +211,58 @@ __device__ __forceinline__ double eval_sdf(const TrajView &tv, const ShapeParams
     return dev::shape_sdf<SHAPE, XFORM>(S, rx, ry);
 }
 
+// getScale (sw_manager.hpp:495-507, the reference's edit point) as svsdf_set_scale specifies it: S(t) = diag(sx, sy, 1),
+// per axis s = c, then s = s + sin(w_k t + phi_k) a_k, at ABSOLUTE time t.  Returns the two diagonal entries of S^-1 as the
+// reference's 3x3 inverse forms them (cofactors times 1/det, Eigen's formula): det = sy sx, S^-1 = diag(sy inv, sx inv, .)
+// with inv = 1 / det — not 1 / sx.  Every other term of the cofactor expansion is a product with an exact zero.
+__device__ __forceinline__ void scale_inv(const ScaleParams &Z, double t, double &i00, double &i11) {
+    double s[2];
+#pragma unroll
+    for (int ax = 0; ax < 2; ++ax) {
+        double v = Z.c[ax];
+#pragma unroll 1
+        for (int k = 0; k < Z.n[ax]; ++k) {
+            double sn, cs;
+            dev::sincos_portable(Z.w[ax][k] * t + Z.phi[ax][k], sn, cs);
+            v = v + sn * Z.a[ax][k];
+        }
+        s[ax] = v;
+    }
+    const double inv = 1.0 / (s[1] * s[0]);
+    i00 = s[1] * inv;
+    i11 = s[0] * inv;
+}
+// posEva2Rel(p, x, R, S) (sw_manager.hpp:528-535): rel = (R^T S^-1) (p - x), the 3x3 product formed first; its zero terms
+// dropped.  With S = I (i00 = i11 = 1 exactly) this is rel_from_pose bit for bit.
+__device__ __forceinline__ void rel_from_pose_scaled(double px, double py, double x, double y, double cy, double sy, double i00,
+                                                     double i11, double &rx, double &ry) {
+    double d0 = px - x, d1 = py - y;
+    rx = (cy * i00) * d0 + (sy * i11) * d1;
+    ry = (-(sy * i00)) * d0 + (cy * i11) * d1;
+}
+// the body-frame point of the scaled body at t (getStateOnTrajStamp(t, xt, Rt, St) + posEva2Rel(p, x, R, S): the rel of
+// getSDFAtTimeStamp<true>, getSDFAtTimeStamp_igl<true> and getGradPrelAtTimeStamp<true>, sw_manager.hpp:741-795).  t is
+// absolute trajectory time.
+__device__ __forceinline__ void rel_at_scaled(const TrajView &tv, const ScaleParams &Z, double px, double py, double t, int &hint,
+                                              double &rx, double &ry) {
+    double x, y, yaw, sy, cy, i00, i11;
+    const double ta = t;
+    const int i = locate_piece(tv, t, hint);
+    traj_pos_at(tv, i, t, x, y, yaw);
+    dev::sincos_portable(yaw, sy, cy);
+    scale_inv(Z, ta, i00, i11);
+    rel_from_pose_scaled(px, py, x, y, cy, sy, i00, i11, rx, ry);
+}
+// the descent's samples: getSDFAtTimeStamp<useScale> (gradientDescent, sw_manager.hpp:1289-1304)
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ double eval_sdf(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, double px, double py,
+                                           double t, int &hint) {
+    if (!SCALED) return eval_sdf<SHAPE, XFORM>(tv, S, px, py, t, hint);
+    double rx, ry;
+    rel_at_scaled(tv, Z, px, py, t, hint, rx, ry);
+    return dev::shape_sdf<SHAPE, XFORM>(S, rx, ry);
+}
+
 // Warp arg-min with the sequential loop's semantics: the FIRST lane holding the minimum value wins; NaN never wins
 // (callers map NaN to +inf; the reference's test is `dis < min_dis`).  Two 32-bit REDUX.MIN over an order-preserving
 // integer image of the double, then a ballot for the first lane.  Returns the winning lane; f becomes the minimum.
@@ -244,9 +296,13 @@ struct OuterResult {
 //   M_M    29 halvings in the actual direction after a misprediction
 // Decisions are the sequential loop's: the slope's sign always comes from the finite difference on lanes 30/31, and the
 // accepted halving is the first (largest step) whose candidate decreases f.
-template <int SHAPE, bool XFORM>
-__device__ __forceinline__ OuterResult solve_outer(const TrajView &tv, const ShapeParams &S, double px, double py,
-                                                   bool have_seed = false, double seed_in = 0.0, double min_in = 1e9) {
+// SCALED: choiceTInit stays rigid whatever useScale says (its four layers call the rigid posEva2Rel, :569-570); the
+// descent evaluates the scaled body, so f(x0) is not choiceTInit's minimum and is evaluated first (M_F0), as the reference
+// does at iter == 0.
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ OuterResult solve_outer(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, double px,
+                                                   double py, bool have_seed = false, double seed_in = 0.0,
+                                                   double min_in = 1e9) {
     const int lane = threadIdx.x & 31;
     const double D = tv.D;
     const double INF = __longlong_as_double(0x7ff0000000000000LL);
@@ -354,8 +410,8 @@ __device__ __forceinline__ OuterResult solve_outer(const TrajView &tv, const Sha
     int mode;
     int tau_hi;        // this lane's step, high word
     unsigned sbit;     // this lane's offset sign bit
-    if (__any_sync(FULL, min_dis >= 1e9)) {
-        // nothing below the initial 1e9 (degenerate input): the reference evaluates f(x0) at iter == 0
+    if (SCALED || __any_sync(FULL, min_dis >= 1e9)) {
+        // nothing below the initial 1e9 (degenerate input), or a scaled body: the reference evaluates f(x0) at iter == 0
         mode = M_F0;
         tau_hi = 0; sbit = 0;   // offset +0.0: the sample is x itself
     } else {
@@ -369,7 +425,7 @@ __device__ __forceinline__ OuterResult solve_outer(const TrajView &tv, const Sha
     while (running) {
         const double off = __hiloint2double(tau_hi ^ (int)sbit, (mode == M_F0) ? 0 : tau_lo);
         const double tq = smaxd(smind(x + off, hi_l), lo_l);
-        const double fq = eval_sdf<SHAPE, XFORM>(tv, S, px, py, tq, hint);
+        const double fq = eval_sdf<SHAPE, XFORM, SCALED>(tv, S, Z, px, py, tq, hint);
         const unsigned m_dec = __ballot_sync(FULL, (fq - fx) < 0);  // candidates that decrease f
         int jacc = -1, src = 0;
         bool failed = false, step_end = true;
@@ -450,14 +506,20 @@ __device__ __forceinline__ OuterResult solve_outer(const TrajView &tv, const Sha
 
 // getGradPrelAtTimeStamp (sw_manager.hpp:779-795) -> getonlyGrad1: central FD, dx = 1e-6 in the body frame
 // (Shape.hpp:35-53), or the Polygon's analytic override (Shape.hpp:1508-1534). 4 lanes do the 4 evaluations.
-template <int SHAPE, bool XFORM>
-__device__ __forceinline__ void grad_prel(const TrajView &tv, const ShapeParams &S, double px, double py, double t,
-                                          double &gx, double &gy) {
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ void grad_prel(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, double px, double py,
+                                          double t, double &gx, double &gy) {
     const int lane = threadIdx.x & 31;
-    double x, y, yaw, sy, cy, rx, ry;
-    traj_pos(tv, t, x, y, yaw);
-    dev::sincos_portable(yaw, sy, cy);
-    rel_from_pose(px, py, x, y, cy, sy, rx, ry);
+    double rx, ry;
+    if (SCALED) {
+        int hint = 0;
+        rel_at_scaled(tv, Z, px, py, t, hint, rx, ry);
+    } else {
+        double x, y, yaw, sy, cy;
+        traj_pos(tv, t, x, y, yaw);
+        dev::sincos_portable(yaw, sy, cy);
+        rel_from_pose(px, py, x, y, cy, sy, rx, ry);
+    }
     if (SHAPE == SH_POLYGON) {
         dev::PolyHit H = dev::polygon_scan(S, rx, ry);
         double vx = rx - H.cx, vy = ry - H.cy;
@@ -514,8 +576,11 @@ struct Contribution {
     double gdT, pena;
     bool active;
 };
-__device__ __forceinline__ Contribution point_contribution(const TrajView &tv, const CostParams &cp, double px,
-                                                           double py, double sdf, double tstar, double gx,
+// SCALED (St = getScale(t*), :827): the xy part is -L' (-S^-T R g); the yaw part keeps the reference's g^T VR^T (p - x),
+// which misses the S^-1 of the true derivative, unless Z.exact_yaw_grad asks for g^T VR^T S^-1 (p - x).
+template <bool SCALED>
+__device__ __forceinline__ Contribution point_contribution(const TrajView &tv, const CostParams &cp, const ScaleParams &Z,
+                                                           double px, double py, double sdf, double tstar, double gx,
                                                            double gy) {
     Contribution C;
     double tl = tstar;
@@ -552,10 +617,14 @@ __device__ __forceinline__ Contribution point_contribution(const TrajView &tv, c
     C.pena = 0.0;
     C.active = false;
     if (sdf_cost > 0) {
-        double rg0 = -(cy * gx + (-sy) * gy);
-        double rg1 = -(sy * gx + cy * gy);
+        double i00 = 1.0, i11 = 1.0;
+        if (SCALED) scale_inv(Z, tstar, i00, i11);
+        // (-S^-T R) g: rows -(i00 c, -i00 s), -(i11 s, i11 c)
+        double rg0 = SCALED ? -((i00 * cy) * gx + (-(i00 * sy)) * gy) : -(cy * gx + (-sy) * gy);
+        double rg1 = SCALED ? -((i11 * sy) * gx + (i11 * cy) * gy) : -(sy * gx + cy * gy);
         double sg0 = -sdf_out_grad * rg0, sg1 = -sdf_out_grad * rg1;
         double d0 = px - pos[0], d1 = py - pos[1];
+        if (SCALED && Z.exact_yaw_grad) { d0 = i00 * d0; d1 = i11 * d1; }
         double w0 = -sy * d0 + cy * d1;
         double w1 = -cy * d0 + -sy * d1;
         double gyaw = (-sdf_out_grad * gx) * w0 + (-sdf_out_grad * gy) * w1;
@@ -652,13 +721,19 @@ __device__ __forceinline__ void thread_choice_t_init(const TrajView &tv, const S
 }
 
 // getGradPrelAtTimeStamp (sw_manager.hpp:779-795) -> getonlyGrad1 (Shape.hpp:35-53), one point per thread
-template <int SHAPE, bool XFORM>
-__device__ __forceinline__ void thread_grad_prel(const TrajView &tv, const ShapeParams &S, double px, double py, double t,
-                                                 double &gx, double &gy) {
-    double x, y, yaw, sy, cy, rx, ry;
-    traj_pos(tv, t, x, y, yaw);
-    dev::sincos_portable(yaw, sy, cy);
-    rel_from_pose(px, py, x, y, cy, sy, rx, ry);
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ void thread_grad_prel(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, double px,
+                                                 double py, double t, double &gx, double &gy) {
+    double rx, ry;
+    if (SCALED) {
+        int hint = 0;
+        rel_at_scaled(tv, Z, px, py, t, hint, rx, ry);
+    } else {
+        double x, y, yaw, sy, cy;
+        traj_pos(tv, t, x, y, yaw);
+        dev::sincos_portable(yaw, sy, cy);
+        rel_from_pose(px, py, x, y, cy, sy, rx, ry);
+    }
     if (SHAPE == SH_POLYGON) {
         dev::PolyHit H = dev::polygon_scan(S, rx, ry);
         double vx = rx - H.cx, vy = ry - H.cy;
@@ -710,8 +785,8 @@ __device__ __forceinline__ void thread_grad_prel(const TrajView &tv, const Shape
 // decreases f, the sign comes from the finite difference — bit-identical results (GPU parity tests, strict build).
 // In: lane i (< nb) holds point i of the batch (px, py, choiceTInit seed and minimum).  Out: res[2 i] = sdf, res[2 i + 1] = t*.
 // ------------------------------------------------------------------------------------------------
-template <int SHAPE, bool XFORM>
-__device__ __forceinline__ void descent_engine(const TrajView &tv, const ShapeParams &S, int nb, double mpx, double mpy,
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ void descent_engine(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, int nb, double mpx, double mpy,
                                                double mseed, double mmin, double *res, unsigned &evals) {
     enum { E_F0 = 0, E_R1 = 1, E_RN = 2 };
     const int lane = threadIdx.x & 31, q = lane & 7, qbase = lane & 24;
@@ -744,7 +819,7 @@ __device__ __forceinline__ void descent_engine(const TrajView &tv, const ShapePa
                     t_min = smaxd(0.0, nsd - 3.4);      // :856-857
                     t_max = smind(nsd + 3.4, D);
                     iter = 0; pred = 1; sgn = 1; jbase = 0; hint = 0;
-                    mode = (nmn >= 1e9) ? E_F0 : E_R1;
+                    mode = (SCALED || nmn >= 1e9) ? E_F0 : E_R1;
                 }
             }
         }
@@ -765,7 +840,7 @@ __device__ __forceinline__ void descent_engine(const TrajView &tv, const ShapePa
         const double hi_l = slope ? ((q == 0) ? INF : D) : t_max;
         const double tc = smaxd(smind(x + off, hi_l), lo_l);
         const double tq = (cand || slope) ? tc : x;
-        const double fq = eval_sdf<SHAPE, XFORM>(tv, S, px, py, tq, hint);
+        const double fq = eval_sdf<SHAPE, XFORM, SCALED>(tv, S, Z, px, py, tq, hint);
 
         // ---- collectives (all lanes), then each quarter's decision, again without branches ----
         const unsigned m8 = (__ballot_sync(FULL, (fq - fx) < 0) >> qbase) & 0xffu;
@@ -816,8 +891,8 @@ __device__ __forceinline__ void descent_engine(const TrajView &tv, const ShapePa
 // wk[4 (32 w + i)], valid for i < nbw[w]; served in the order i-major, w-minor through the shared cursor): a group that
 // finishes its point takes the next one of the whole CTA, so the warps of a CTA finish together whatever the lengths of
 // their own descents.  Which group solves a point does not change its result; the reductions stay per warp, fixed order.
-template <int SHAPE, bool XFORM>
-__device__ __forceinline__ void descent_engine2(const TrajView &tv, const ShapeParams &S, double *wk, const int *nbw, int *cursor,
+template <int SHAPE, bool XFORM, bool SCALED>
+__device__ __forceinline__ void descent_engine2(const TrajView &tv, const ShapeParams &S, const ScaleParams &Z, double *wk, const int *nbw, int *cursor,
                                                 int limit, unsigned &evals) {
     enum { E_F0 = 0, E_R1 = 1, E_RN = 2 };
     const int lane = threadIdx.x & 31, q = lane & 3, gbase = lane & 28;
@@ -849,7 +924,7 @@ __device__ __forceinline__ void descent_engine2(const TrajView &tv, const ShapeP
                     t_min = smaxd(0.0, nsd - 3.4);
                     t_max = smind(nsd + 3.4, D);
                     iter = 0; pred = 1; sgn = 1; jbase = 0; hintA = 0; hintB = 0;
-                    mode = (nmn >= 1e9) ? E_F0 : E_R1;
+                    mode = (SCALED || nmn >= 1e9) ? E_F0 : E_R1;   // scaled: f(x0) is not choiceTInit's minimum
                 }
             }
         }
@@ -872,8 +947,8 @@ __device__ __forceinline__ void descent_engine2(const TrajView &tv, const ShapeP
         const double loA = slopeA ? ((q == 0) ? 0.0 : -INF) : t_min, hiA = slopeA ? ((q == 0) ? INF : D) : t_max;
         const double tcA = smaxd(smind(x + offA, hiA), loA), tcB = smaxd(smind(x + offB, t_max), t_min);
         const double tA = (candA || slopeA) ? tcA : x, tB = candB ? tcB : x;
-        const double fA = eval_sdf<SHAPE, XFORM>(tv, S, px, py, tA, hintA);
-        const double fB = eval_sdf<SHAPE, XFORM>(tv, S, px, py, tB, hintB);
+        const double fA = eval_sdf<SHAPE, XFORM, SCALED>(tv, S, Z, px, py, tA, hintA);
+        const double fB = eval_sdf<SHAPE, XFORM, SCALED>(tv, S, Z, px, py, tB, hintB);
 
         const unsigned balA = __ballot_sync(FULL, (fA - fx) < 0), balB = __ballot_sync(FULL, (fB - fx) < 0);
         const unsigned m8 = ((balA >> gbase) & 0xfu) | (((balB >> gbase) & 0xfu) << 4);
@@ -983,9 +1058,11 @@ __global__ void k_pose_table(double *blob) {
 #define SVSDF_GSIP_MIN_CTAS 3
 #endif
 // BATCHED selects the schedule at compile time (two kernels: each carries only its own evaluation sites)
-template <int SHAPE, bool XFORM, bool BATCHED>
+// SCALED: the body scale S(t) of svsdf_set_scale (Z) on every evaluation after choiceTInit (only the batched schedule is
+// instantiated scaled)
+template <int SHAPE, bool XFORM, bool BATCHED, bool SCALED>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, (SHAPE == SH_MESH) ? SVSDF_MESH_MIN_CTAS : SVSDF_OUTER_MIN_CTAS)
-    k_outer(const __grid_constant__ KernelArgs A, const __grid_constant__ ShapeParams S) {
+    k_outer(const __grid_constant__ KernelArgs A, const __grid_constant__ ShapeParams S, const __grid_constant__ ScaleParams Z) {
     extern __shared__ __align__(16) double smem[];
     __shared__ __align__(8) uint64_t bar;
     __shared__ int s_nb[kWarpsPerBlock];
@@ -1036,11 +1113,11 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, (SHAPE == SH_MESH) ? SVSD
             if (lane == 0) s_nb[warp] = nb;
             if (threadIdx.x == 0) s_cursor = 0;
             __syncthreads();   // every warp has the same number of batches (nB is a multiple of the warp count)
-            descent_engine2<SHAPE, XFORM>(tv, S, res - 128 * warp, s_nb, &s_cursor, kWarpsPerBlock * 32, ev2);
+            descent_engine2<SHAPE, XFORM, SCALED>(tv, S, Z, res - 128 * warp, s_nb, &s_cursor, kWarpsPerBlock * 32, ev2);
             __syncthreads();
             if (my_valid) { m_sdf = res[4 * lane]; m_ts = res[4 * lane + 1]; }
 #else
-            descent_engine<SHAPE, XFORM>(tv, S, nb, mpx, mpy, m_seed, m_min, res, ev2);
+            descent_engine<SHAPE, XFORM, SCALED>(tv, S, Z, nb, mpx, mpy, m_seed, m_min, res, ev2);
             if (my_valid) { m_sdf = res[2 * lane]; m_ts = res[2 * lane + 1]; }
 #endif
             my_evals += (unsigned long long)__reduce_add_sync(FULL, (unsigned)ev + ev2);
@@ -1049,16 +1126,16 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, (SHAPE == SH_MESH) ? SVSD
 #pragma unroll 1
             for (int i = 0; i < nb; ++i) {
                 const double px = __shfl_sync(FULL, mpx, i), py = __shfl_sync(FULL, mpy, i);
-                const OuterResult R = solve_outer<SHAPE, XFORM>(tv, S, px, py);
+                const OuterResult R = solve_outer<SHAPE, XFORM, SCALED>(tv, S, Z, px, py);
                 my_evals += (unsigned long long)R.evals;
                 if (lane == i) { m_sdf = R.sdf; m_ts = R.tstar; }
                 double gx, gy;
-                grad_prel<SHAPE, XFORM>(tv, S, px, py, R.tstar, gx, gy);
+                grad_prel<SHAPE, XFORM, SCALED>(tv, S, Z, px, py, R.tstar, gx, gy);
                 if (lane == i) { m_gx = gx; m_gy = gy; }
             }
         }
         my_evals += 4ull * (unsigned long long)nb;
-        if (BATCHED && batched && my_valid) thread_grad_prel<SHAPE, XFORM>(tv, S, mpx, mpy, m_ts, m_gx, m_gy);
+        if (BATCHED && batched && my_valid) thread_grad_prel<SHAPE, XFORM, SCALED>(tv, S, Z, mpx, mpy, m_ts, m_gx, m_gy);
         // ---- per-lane epilogue: outputs, interior flag, penalty + chain rule (one point per lane) ----
         const bool inside = my_valid && A.want_gsip && !(m_sdf > 0);  // getTrueSDFofSweptVolume: `if (argmin_dis > 0) return`
         if (my_valid) {
@@ -1072,7 +1149,7 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, (SHAPE == SH_MESH) ? SVSD
         if (A.want_reduce) {
             Contribution C;
             C.active = false;
-            if (my_valid && !inside) C = point_contribution(tv, A.cp, mpx, mpy, m_sdf, m_ts, m_gx, m_gy);
+            if (my_valid && !inside) C = point_contribution<SCALED>(tv, A.cp, Z, mpx, mpy, m_sdf, m_ts, m_gx, m_gy);
             // accumulate the active lanes' contributions in batch order (deterministic)
             unsigned m = __ballot_sync(FULL, C.active);
             while (m) {
@@ -1174,9 +1251,10 @@ __global__ void __launch_bounds__(1024) k_compact(const unsigned char *flag, int
 // running a full outer solve on its sample.
 // dynamic smem: [ blob ]
 // ------------------------------------------------------------------------------------------------
-template <int SHAPE, bool XFORM, int WARPS>
+// SCALED: the ring samples' outer solves and the chain rule use S(t) (only the 8-warp width is instantiated scaled)
+template <int SHAPE, bool XFORM, int WARPS, bool SCALED>
 __global__ void __launch_bounds__(WARPS * 32, (WARPS == kWarpsPerBlock && SHAPE != SH_MESH) ? SVSDF_GSIP_MIN_CTAS : 1)
-    k_gsip(const __grid_constant__ KernelArgs A, const __grid_constant__ ShapeParams S) {
+    k_gsip(const __grid_constant__ KernelArgs A, const __grid_constant__ ShapeParams S, const __grid_constant__ ScaleParams Z) {
     extern __shared__ __align__(16) double smem[];
     __shared__ __align__(8) uint64_t bar;
     __shared__ double s_theta[24], s_val[24], s_ts[24];
@@ -1229,7 +1307,7 @@ __global__ void __launch_bounds__(WARPS * 32, (WARPS == kWarpsPerBlock && SHAPE 
                 double sn, cs;
                 dev::sincos_portable(th, sn, cs);
                 double yx = px + 1.0 * r * cs, yy = py + 1.0 * r * sn;  // CircleCoord2D::getPosition (:36-39)
-                OuterResult R = solve_outer<SHAPE, XFORM>(tv, S, yx, yy);
+                OuterResult R = solve_outer<SHAPE, XFORM, SCALED>(tv, S, Z, yx, yy);
                 my_evals += (unsigned long long)R.evals;
                 if (lane == 0) { s_val[k] = R.sdf; s_ts[k] = R.tstar; }
             }
@@ -1271,7 +1349,7 @@ __global__ void __launch_bounds__(WARPS * 32, (WARPS == kWarpsPerBlock && SHAPE 
             if (A.out_rounds) A.out_rounds[pt] = rounds;
         }
         if (A.want_reduce && warp == 0) {
-            Contribution C = point_contribution(tv, A.cp, px, py, sdf, real_t_star, gx, gy);
+            Contribution C = point_contribution<SCALED>(tv, A.cp, Z, px, py, sdf, real_t_star, gx, gy);
             double *o = A.gsip_contrib + 20 * (int64_t)slot;
             if (lane < 18) {
                 int d = lane / 6, q = lane - 6 * d;
@@ -1427,37 +1505,71 @@ struct LaunchCfg {
     cudaStream_t stream;
     cudaEvent_t after_outer;  // optional timing mark recorded right after k_outer
     bool gsip_wide;           // use the 22-warp k_gsip variant
+    const ScaleParams *scale; // body scale S(t) (null: rigid body)
 };
+
+// Scaled body: one k_outer schedule (batched: correct for every P) and one k_gsip width, so that the scale adds two
+// instantiations per shape instead of four.
+template <int SHAPE, bool XFORM>
+static cudaError_t launch_shape_scaled(const KernelArgs &A, const ShapeParams &S, const LaunchCfg &cfg) {
+    cudaError_t e;
+    static bool attr_set_dev[64] = {};
+    int dev_ord = 0;
+    cudaGetDevice(&dev_ord);
+    bool &attr_set = attr_set_dev[dev_ord & 63];
+    if (!attr_set) {
+        e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kWarpsPerBlock, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e != cudaSuccess) return e;
+        attr_set = true;
+    }
+    KernelArgs B = A;
+    B.batched = 1;
+    k_outer<SHAPE, XFORM, true, true><<<cfg.grid_outer, kWarpsPerBlock * 32, cfg.smem_outer, cfg.stream>>>(B, S, *cfg.scale);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    if (cfg.after_outer) cudaEventRecord(cfg.after_outer, cfg.stream);
+    if (A.want_gsip) {
+        k_compact<<<1, 1024, 0, cfg.stream>>>(A.inside_flag, A.P, A.inside_list, A.n_inside);
+        k_gsip<SHAPE, XFORM, kWarpsPerBlock, true><<<cfg.grid_gsip, kWarpsPerBlock * 32, cfg.smem_gsip, cfg.stream>>>(B, S, *cfg.scale);
+        e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
 
 template <int SHAPE, bool XFORM>
 static cudaError_t launch_shape(const KernelArgs &A, const ShapeParams &S, const LaunchCfg &cfg, int N) {
+    if (cfg.scale) return launch_shape_scaled<SHAPE, XFORM>(A, S, cfg);
     cudaError_t e;
+    const ScaleParams Z{};
     // the attribute is per device (a process may hold contexts on several GPUs): one flag per device ordinal
     static bool attr_set_dev[64] = {};
     int dev_ord = 0;
     cudaGetDevice(&dev_ord);
     bool &attr_set = attr_set_dev[dev_ord & 63];
     if (!attr_set) {
-        e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kWarpsPerBlock>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kWarpsPerBlock, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kGsipWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kGsipWarps, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
         attr_set = true;
     }
-    if (A.batched) k_outer<SHAPE, XFORM, true><<<cfg.grid_outer, kWarpsPerBlock * 32, cfg.smem_outer, cfg.stream>>>(A, S);
-    else k_outer<SHAPE, XFORM, false><<<cfg.grid_outer, kWarpsPerBlock * 32, cfg.smem_outer, cfg.stream>>>(A, S);
+    if (A.batched) k_outer<SHAPE, XFORM, true, false><<<cfg.grid_outer, kWarpsPerBlock * 32, cfg.smem_outer, cfg.stream>>>(A, S, Z);
+    else k_outer<SHAPE, XFORM, false, false><<<cfg.grid_outer, kWarpsPerBlock * 32, cfg.smem_outer, cfg.stream>>>(A, S, Z);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     if (cfg.after_outer) cudaEventRecord(cfg.after_outer, cfg.stream);
     if (A.want_gsip) {
         k_compact<<<1, 1024, 0, cfg.stream>>>(A.inside_flag, A.P, A.inside_list, A.n_inside);
         // few inside points: one warp per ring sample (latency); many: 8-warp CTAs, two per SM (throughput)
-        if (cfg.gsip_wide) k_gsip<SHAPE, XFORM, kGsipWarps><<<cfg.grid_gsip, kGsipWarps * 32, cfg.smem_gsip, cfg.stream>>>(A, S);
-        else k_gsip<SHAPE, XFORM, kWarpsPerBlock><<<cfg.grid_gsip, kWarpsPerBlock * 32, cfg.smem_gsip, cfg.stream>>>(A, S);
+        if (cfg.gsip_wide) k_gsip<SHAPE, XFORM, kGsipWarps, false><<<cfg.grid_gsip, kGsipWarps * 32, cfg.smem_gsip, cfg.stream>>>(A, S, Z);
+        else k_gsip<SHAPE, XFORM, kWarpsPerBlock, false><<<cfg.grid_gsip, kWarpsPerBlock * 32, cfg.smem_gsip, cfg.stream>>>(A, S, Z);
         e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
@@ -1496,16 +1608,17 @@ static cudaError_t dispatch(const KernelArgs &A, const ShapeParams &S, const Lau
 
 template <int SHAPE, bool XFORM>
 static cudaError_t occ_shape(size_t smem_outer, size_t smem_gsip, int *occ_outer, int *occ_gsip) {
-    cudaError_t e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    e = cudaFuncSetAttribute(k_outer<SHAPE, XFORM, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kWarpsPerBlock>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    e = cudaFuncSetAttribute(k_gsip<SHAPE, XFORM, kWarpsPerBlock, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return e;
-    // the two schedules are compiled to the same register cap (launch bounds); the batched kernel sizes the full wave
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ_outer, k_outer<SHAPE, XFORM, true>, kWarpsPerBlock * 32, smem_outer);
+    // the two schedules are compiled to the same register cap (launch bounds); the batched kernel sizes the full wave.  The
+    // scaled instantiations have the same launch bounds and shared memory, so the rigid figures size their grids too.
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ_outer, k_outer<SHAPE, XFORM, true, false>, kWarpsPerBlock * 32, smem_outer);
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ_gsip, k_gsip<SHAPE, XFORM, kWarpsPerBlock>, kWarpsPerBlock * 32, smem_gsip);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ_gsip, k_gsip<SHAPE, XFORM, kWarpsPerBlock, false>, kWarpsPerBlock * 32, smem_gsip);
 }
 
 // Resident CTAs per SM of k_outer / k_gsip for this shape and trajectory size: the host sizes the grids as
@@ -1546,9 +1659,10 @@ cudaError_t launch_pose_table(double *blob, int K1, cudaStream_t stream) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_cost_kernels(const KernelArgs &A, const ShapeParams &S, int N, int grid_outer, int grid_gsip,
-                                cudaStream_t stream, cudaEvent_t after_outer, int gsip_wide) {
+cudaError_t launch_cost_kernels(const KernelArgs &A, const ShapeParams &S, const ScaleParams *scale, int N, int grid_outer,
+                                int grid_gsip, cudaStream_t stream, cudaEvent_t after_outer, int gsip_wide) {
     LaunchCfg cfg;
+    cfg.scale = scale;
     cfg.after_outer = after_outer;
     cfg.gsip_wide = gsip_wide != 0;
     cfg.grid_outer = grid_outer;

@@ -10,8 +10,8 @@ namespace svsdf {
     namespace NS {                                                                                               \
     cudaError_t launch_pose_table(double *blob, int K1, cudaStream_t stream);                                    \
     cudaError_t query_occupancy(const ShapeParams &S, int N, int blob_doubles, int *occ_outer, int *occ_gsip);   \
-    cudaError_t launch_cost_kernels(const KernelArgs &A, const ShapeParams &S, int N, int grid_outer,            \
-                                    int grid_gsip, cudaStream_t stream, cudaEvent_t after_outer,                 \
+    cudaError_t launch_cost_kernels(const KernelArgs &A, const ShapeParams &S, const ScaleParams *scale, int N,  \
+                                    int grid_outer, int grid_gsip, cudaStream_t stream, cudaEvent_t after_outer, \
                                     int gsip_wide);                                                              \
     cudaError_t launch_finalize(const double *partials, int n_blocks, int N, const int *n_inside,                \
                                 const double *gsip_contrib, const int *gsip_piece, double *tot,                  \

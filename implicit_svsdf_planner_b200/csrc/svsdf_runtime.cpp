@@ -38,6 +38,8 @@ struct svsdf_ctx {
     std::string shape_name;
     ShapeParams shape;
     CostParams cp;
+    bool scaled = false;  // svsdf_set_scale: body scale S(t) on the cost path (false: rigid body)
+    ScaleParams scale{};
     double rho = 3.8;
     int device = 0;
     bool strict = false;
@@ -425,7 +427,8 @@ int run_kernels(svsdf_ctx *ctx, const double *d_points, int64_t P, bool reduce, 
     A.gsip_piece = ctx->d_gsip_piece;
     A.eval_counter = ctx->count_evals ? ctx->d_eval_counter : nullptr;
     // previous evaluation had few interior points -> 22-warp CTAs (one warp per ring sample, lower latency)
-    const int gsip_wide = (reduce && ctx->last_n_inside >= 0 && ctx->last_n_inside <= ctx->sm_count) ? 1 : 0;
+    // (the scaled kernels exist in the 8-warp width only)
+    const int gsip_wide = (!ctx->scaled && reduce && ctx->last_n_inside >= 0 && ctx->last_n_inside <= ctx->sm_count) ? 1 : 0;
     const int grid_gsip = gsip_wide ? ctx->sm_count : ctx->sm_count * ctx->occ_gsip;
     if (!gsip) CK(cudaMemsetAsync(ctx->d_n_inside, 0, sizeof(int), ctx->stream));
     size_t smem = outer_smem_doubles(A.blob_doubles, N) * sizeof(double);
@@ -433,9 +436,10 @@ int run_kernels(svsdf_ctx *ctx, const double *d_points, int64_t P, bool reduce, 
         ctx->err = "svsdf: trajectory blob does not fit in shared memory";
         return SVSDF_ERR_INVALID;
     }
-    cudaError_t e = ctx->strict ? strict::launch_cost_kernels(A, ctx->shape, N, grid, grid_gsip, ctx->stream,
+    const ScaleParams *Z = ctx->scaled ? &ctx->scale : nullptr;
+    cudaError_t e = ctx->strict ? strict::launch_cost_kernels(A, ctx->shape, Z, N, grid, grid_gsip, ctx->stream,
                                                               ctx->mark_kernels ? ctx->evk[2] : nullptr, gsip_wide)
-                                : fast::launch_cost_kernels(A, ctx->shape, N, grid, grid_gsip, ctx->stream,
+                                : fast::launch_cost_kernels(A, ctx->shape, Z, N, grid, grid_gsip, ctx->stream,
                                                             ctx->mark_kernels ? ctx->evk[2] : nullptr, gsip_wide);
     CK(e);
     ctx->launches += gsip ? 3 : 1;
@@ -1283,6 +1287,51 @@ int svsdf_device_ptr_points(svsdf_ctx *ctx, const double **dev_xy) {
         ctx->pts_inflight = false;
     }
     *dev_xy = ctx->d_points;
+    return SVSDF_OK;
+}
+
+int svsdf_set_scale(svsdf_ctx *ctx, const svsdf_scale *spec) {
+    if (!ctx) return SVSDF_ERR_INVALID;
+    if (!spec) {
+        ctx->scaled = false;
+        return SVSDF_OK;
+    }
+    ScaleParams Z{};
+    for (int ax = 0; ax < 2; ++ax) {
+        const int n = spec->n_terms[ax];
+        if (n < 0 || n > kMaxScaleTerms) {
+            ctx->err = "svsdf_set_scale: n_terms must be in [0, 4]";
+            return SVSDF_ERR_INVALID;
+        }
+        double amp = 0.0;
+        bool finite = std::isfinite(spec->c[ax]);
+        for (int k = 0; k < n; ++k)
+            finite = finite && std::isfinite(spec->a[ax][k]) && std::isfinite(spec->w[ax][k]) && std::isfinite(spec->phi[ax][k]);
+        if (!finite) {
+            ctx->err = "svsdf_set_scale: non-finite entry";
+            return SVSDF_ERR_INVALID;
+        }
+        for (int k = 0; k < n; ++k) amp += std::fabs(spec->a[ax][k]);
+        // the scale must stay positive at every t: S^-1 is singular where an axis reaches 0
+        if (!(spec->c[ax] - amp > 0.0)) {
+            ctx->err = "svsdf_set_scale: c - sum |a_k| must be > 0 on both axes";
+            return SVSDF_ERR_INVALID;
+        }
+        Z.n[ax] = n;
+        Z.c[ax] = spec->c[ax];
+        for (int k = 0; k < n; ++k) {
+            Z.a[ax][k] = spec->a[ax][k];
+            Z.w[ax][k] = spec->w[ax][k];
+            Z.phi[ax][k] = spec->phi[ax][k];
+        }
+    }
+    if (spec->exact_yaw_grad != 0 && spec->exact_yaw_grad != 1) {
+        ctx->err = "svsdf_set_scale: exact_yaw_grad must be 0 or 1";
+        return SVSDF_ERR_INVALID;
+    }
+    Z.exact_yaw_grad = spec->exact_yaw_grad;
+    ctx->scale = Z;
+    ctx->scaled = true;
     return SVSDF_OK;
 }
 

@@ -119,6 +119,15 @@ struct CostParams {
     double safety_hor;
 };
 
+// Time-varying body scale S(t) = diag(s_x(t), s_y(t), 1) (svsdf_set_scale): per axis
+// s(t) = c, then s = s + sin(w_k t + phi_k) a_k for k < n, in that order; t is absolute trajectory time.
+constexpr int kMaxScaleTerms = 4;
+struct ScaleParams {
+    int n[2];
+    double c[2], a[2][kMaxScaleTerms], w[2][kMaxScaleTerms], phi[2][kMaxScaleTerms];
+    int exact_yaw_grad;  // 0: the reference's yaw term g^T VR^T (p - x); 1: g^T VR^T S^-1 (p - x)
+};
+
 // Kernel argument block
 struct KernelArgs {
     const double *blob;        // trajectory blob (global)

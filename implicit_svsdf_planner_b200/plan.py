@@ -74,8 +74,11 @@ def rot_z(yaw: float) -> np.ndarray:
 
 def generate_traj(ctx: "api.Context", cmap: CloudMap, start_xy, goal_xy, kernel_size: int = scenes.YAML["kernel_size"], kernel_yaw_num: int = 18,
                   front_end_safeh: float = 0.0, traj_parlength: float = 3.0, inittime: float = scenes.YAML["inittime"],
-                  mid_cfg: Optional["api.MidConfig"] = None, lbfgs_params=None, max_path: int = 4096) -> dict:
-    """generatePath + generateTraj for one start / goal on the map `cmap` (the context's shape is the robot)."""
+                  mid_cfg: Optional["api.MidConfig"] = None, lbfgs_params=None, max_path: int = 4096, scale: Optional[dict] = None) -> dict:
+    """generatePath + generateTraj for one start / goal on the map `cmap` (the context's shape is the robot).
+    scale: a deformable robot's body scale for the back end only (keyword arguments of Context.set_scale, e.g.
+    api.REFERENCE_SCALE_EXAMPLE); the front and mid ends plan for the rigid body, as the reference's do.  The context is
+    back to the rigid body when the call returns."""
     X, Y, Z = cmap.occ.shape
     res = cmap.res
     ctx.set_map3d(pack_map_kernel3d(cmap.occ, kernel_size), X, Y, Z, kernel_size, cmap.boundary_min, res)
@@ -95,8 +98,14 @@ def generate_traj(ctx: "api.Context", cmap: CloudMap, start_xy, goal_xy, kernel_
     if rc_mid < 0:
         return dict(ok=False, reason=f"mid end failed ({rc_mid})", N=N, n_points=int(n_points))
     params = lbfgs_params or api.default_lbfgs_params(mem_size=16, past=3, delta=1e-6, g_epsilon=0.0, max_iterations=0, min_step=1e-32)
-    f0, _ = ctx_evaluate(ctx, init_s, final_s, N, opt_x)
-    rc, x, T, b, st = ctx.optimize(init_s, final_s, opt_x, N, params)  # the query points are the context's resident set (extract_points3d)
+    if scale is not None:
+        ctx.set_scale(**scale)
+    try:
+        f0, _ = ctx_evaluate(ctx, init_s, final_s, N, opt_x)
+        rc, x, T, b, st = ctx.optimize(init_s, final_s, opt_x, N, params)  # the query points are the context's resident set (extract_points3d)
+    finally:
+        if scale is not None:
+            ctx.set_scale()
     return dict(ok=rc >= 0, status=int(rc), N=N, n_points=int(n_points), path=path, waypoints=wps, expansions=int(expansions[0]), astar_rounds=int(rounds),
                 mid=dict(status=int(rc_mid), cost=float(cost_mid), iterations=int(it_mid), T=T_mid), cost_at_warm_start=float(f0),
                 final_cost=float(st["final_cost"]), iterations=int(st["iterations"]), evaluations=int(st["evaluations"]), T=T, coeffs=b, x=x,

@@ -108,6 +108,27 @@ int svsdf_set_points_device(svsdf_ctx *ctx, const double *dev_xy, int64_t P);
 /* R2: updateTraj.  T: N durations; coeffs: MINCO `b`, 6N x 3 column-major. */
 int svsdf_set_traj(svsdf_ctx *ctx, int N, const double *T, const double *coeffs);
 
+/* Deformable robot (the reference's useScale switch with its getScale hook, sw_manager.hpp:17, 495-507): the body maps to
+ * the world as p = S(t) R(yaw) q + x, with S(t) = diag(s_x(t), s_y(t), 1) acting along WORLD axes after the rotation (for
+ * s_x = s_y the distinction disappears) and t absolute trajectory time.  Per axis ax (0 = x, 1 = y):
+ *     s = c[ax];  for (k = 0; k < n_terms[ax]; ++k) s = s + sin(w[ax][k] * t + phi[ax][k]) * a[ax][k];
+ * evaluated in exactly that order with the pinned fdlibm sin.  The reference's commented example is n_terms = {1, 1},
+ * (c, a, w, phi) = (0.8, 0.6, 1.5, -1.0) for x and (0.8, 0.4, 1.8, 0.0) for y.
+ * As in the reference, choiceTInit stays rigid; the descent, the body-frame gradient, the interior branch's ring solves and
+ * the chain rule use S(t).  exact_yaw_grad = 0 keeps the reference's yaw term g^T VR^T (p - x) (not the derivative once
+ * S != I); 1 uses the true derivative g^T VR^T S^-1 (p - x). */
+typedef struct {
+    int n_terms[2];   /* 0..4 */
+    double c[2], a[2][4], w[2][4], phi[2][4];
+    int exact_yaw_grad;
+} svsdf_scale;
+/* Applies to this context's svsdf_query, svsdf_cost_grad[_device], svsdf_evaluate, svsdf_optimize and batch entries (each
+ * context of a pool uses its own spec: give every context of a pool the same one).  The front end (svsdf_front_*), the mid end
+ * and svsdf_shape_sdf / _grad1 (body frame) stay rigid, like the reference's.  spec = NULL returns to the rigid body (the
+ * default).  SVSDF_ERR_INVALID (the previous setting is kept) when n_terms is outside [0, 4], an entry in use is not
+ * finite, or c - sum_k |a_k| <= 0 on either axis (the scale must stay positive for S^-1 to exist). */
+int svsdf_set_scale(svsdf_ctx *ctx, const svsdf_scale *spec);
+
 /* R2: per-point swept-volume SDF query on the trajectory given by (N, T, coeffs).
  * pts: P x 3 (x, y, z) host doubles (z ignored).  Outputs (host, may be NULL): sdf[P], tstar[P], grad3[3P]
  * (body-frame FD gradient for sdf > 0; world-frame unit direction for the interior branch, exactly what the

@@ -127,6 +127,9 @@ class SweptVolumeManager {
         N_ = N; T_.assign(T, T + N); c_.assign(coeffs, coeffs + 18 * (size_t)N);
         return svsdf_set_traj(ctx_->h, N, T, coeffs);
     }
+    // `#define useScale true` plus an edited getScale (:17, :495-507): the body scale S(t) as an svsdf_scale spec (see
+    // svsdf.h); nullptr returns to the rigid body.  Returns 0 or SVSDF_ERR_INVALID.
+    int setScale(const svsdf_scale *spec) { return svsdf_set_scale(ctx_->h, spec); }
     // getTrueSDFofSweptVolume<true>(pos_eva, time_seed_f, grad_prel, set_ts) (:916-1018); set_ts is ignored like the reference's
     // call sites pass false (the scan always runs).
     double getTrueSDFofSweptVolume(const double pos_eva[3], double &time_seed_f, double grad_prel[3], bool /*set_ts*/ = false) {
